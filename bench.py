@@ -22,6 +22,15 @@ Haiku-default random weights.  Prints ONE JSON line on rank 0.
   cpu_baseline / --impl reference : the fp32 CPU oracle (torch-CPU) on a bounded sample of the
              SAME workload: a contiguous block of 1/16 of the rows of every stage of the real
              0.25 degree graph (oracle/sampled_step.py), scaled by the row fraction.
+
+--dump-outputs DIR writes what the last headline step returned, so that two builds run with the
+same arguments (hence the same seeded inputs and weights) can be compared output for output:
+  DIR/predictions.npy  float32 [n_out, k]: the step's output planes at k grid nodes (all of
+                       them when they fit in 32 MiB, else a fixed seeded sample)
+  DIR/grid_index.npy   float64 [k]: the grid node index of each column
+
+The source tree may be read-only: nothing is written there (no bytecode; the static-graph cache
+goes to a per-user temporary directory unless GRAPHCAST_B200_CACHE says otherwise).
 """
 
 import argparse
@@ -30,6 +39,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -54,6 +64,7 @@ WORKLOADS = {
 }
 DEFAULT_WORKLOAD = "graphcast_0.25deg_37lvl"
 REFERENCE_BUDGET_S = 150.0   # wall-clock target of a whole `--impl reference` run
+DUMP_BYTES = 32 << 20        # --dump-outputs: size of the sampled output (the full 0.25 deg one is 943 MB)
 
 
 def algorithmic_flops(ng, nm, e1, e2, e3, c_in, n_out, steps, d=512):
@@ -242,6 +253,19 @@ def ncu_traffic(workload, precision):
   return tc, f"ncu, profiles/r02_launches_ncu.csv (whole step {total / 1e9:.1f} GB)"
 
 
+def dump_outputs(out_dir, planes_out):
+  """Writes the step output planes_out [n_out, Ng] (device, fp32) to out_dir: every grid node if
+  it fits in DUMP_BYTES, else the same seeded sample of grid nodes on every run."""
+  import torch
+  n_out, ng = planes_out.shape
+  k = min(ng, DUMP_BYTES // (4 * n_out + 8))
+  idx = np.arange(ng) if k == ng else np.sort(np.random.default_rng(0).choice(ng, k, replace=False))
+  sample = planes_out.index_select(1, torch.as_tensor(idx, device=planes_out.device))
+  os.makedirs(out_dir, exist_ok=True)
+  np.save(os.path.join(out_dir, "predictions.npy"), sample.cpu().numpy())
+  np.save(os.path.join(out_dir, "grid_index.npy"), idx.astype(np.float64))
+
+
 def run_b200(args):
   import torch
   import torch.distributed as dist
@@ -308,6 +332,8 @@ def run_b200(args):
     dist.barrier()
   elapsed_ms = ev0.elapsed_time(ev1)
   clocks = sampler.stop() if rank == 0 else None
+  if args.dump_outputs and rank == 0:
+    dump_outputs(args.dump_outputs, planes_out)
 
   # Profiling pass (separate from the headline): the same loop with a CUDA-event pair around
   # every launch (direct launches instead of graph replay) -> per-kernel durations.
@@ -743,6 +769,10 @@ def main():
   os.dup2(2, 1)
   sys.stdout = os.fdopen(real_stdout, "w", buffering=1)
   os.environ["NCCL_DEBUG"] = os.environ.get("GCB_NCCL_DEBUG", "INFO")   # communicator lines on stderr
+  # The project modules are imported after this point; the tree may be read-only.
+  sys.dont_write_bytecode = True
+  os.environ.setdefault("GRAPHCAST_B200_CACHE",
+                        os.path.join(tempfile.gettempdir(), f"graphcast_b200_cache_{os.getuid()}"))
   ap = argparse.ArgumentParser()
   ap.add_argument("--gpus", type=int, default=1)
   ap.add_argument("--steps", type=int, default=10)
@@ -765,6 +795,8 @@ def main():
   ap.add_argument("--skip-cpu-baseline", action="store_true")
   ap.add_argument("--cluster", type=int, default=0, help="CTAs per cluster (0 = library default)")
   ap.add_argument("--dump-launches", default="", help="write per-launch (kind, ms, GFLOP, GB) of the last timed step to this file")
+  ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                  help="write the output of the last timed step to DIR/*.npy (single-forecast GPU path)")
   ap.add_argument("--no-fuse", dest="fuse", action="store_false",
                   help="one launch per linear layer (hidden activations through HBM)")
   ap.add_argument("--chain-lag", dest="chain_lag", type=int, default=0)
@@ -775,11 +807,17 @@ def main():
   ap.add_argument("--no-pregather", dest="pregather", action="store_false",
                   help="evaluate the first edge-MLP layer over the concatenated K=1536 input")
   args = ap.parse_args()
+  if args.steps < 1:
+    ap.error("--steps must be at least 1")
+  partitioned = args.mode == "partitioned" or (args.mode == "auto" and dist_env()[1] > 1)
+  if args.dump_outputs and (args.impl == "reference" or args.rollout > 0 or partitioned):
+    ap.error("--dump-outputs applies to the single-forecast GPU path (--impl b200, no --rollout, "
+             "--mode replicas for N > 1)")
   if args.impl == "reference":
     run_reference(args)
   elif args.rollout > 0:
     run_rollout(args)
-  elif args.mode == "partitioned" or (args.mode == "auto" and dist_env()[1] > 1):
+  elif partitioned:
     run_partitioned(args)
   else:
     run_b200(args)

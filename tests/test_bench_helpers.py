@@ -43,3 +43,25 @@ def test_algorithmic_flops_match_the_survey():
   import bench
   f = bench.algorithmic_flops(1038240, 40962, 1618818, 327660, 3114720, 471, 227, 16)
   assert abs(f / 1e12 - 29.29) < 0.01                     # SURVEY.md section 8(d)
+
+
+def test_dump_outputs_writes_the_whole_output_or_a_fixed_sample(bench, tmp_path, monkeypatch):
+  import numpy as np
+  import torch
+  planes = torch.randn(7, 1000)
+  bench.dump_outputs(str(tmp_path / "all"), planes)
+  np.testing.assert_array_equal(np.load(tmp_path / "all" / "predictions.npy"), planes.numpy())
+  np.testing.assert_array_equal(np.load(tmp_path / "all" / "grid_index.npy"), np.arange(1000))
+
+  monkeypatch.setattr(bench, "DUMP_BYTES", 4096)
+  for run in ("a", "b"):
+    bench.dump_outputs(str(tmp_path / run), planes)
+  files = {run: {n: np.load(tmp_path / run / f"{n}.npy") for n in ("predictions", "grid_index")}
+           for run in ("a", "b")}
+  idx, pred = files["a"]["grid_index"], files["a"]["predictions"]
+  assert idx.dtype == np.float64 and pred.dtype == np.float32
+  assert pred.nbytes + idx.nbytes <= 4096 and pred.shape == (7, idx.size) and idx.size > 100
+  assert np.all(np.diff(idx) > 0)
+  np.testing.assert_array_equal(pred, planes.numpy()[:, idx.astype(np.int64)])
+  np.testing.assert_array_equal(files["b"]["grid_index"], idx)
+  np.testing.assert_array_equal(files["b"]["predictions"], pred)
