@@ -136,6 +136,8 @@ int validate_layer(const gcb_layer_desc* d) {
   if (d->out_y) GCB_CHECK_ARG(aligned16(d->out_y) && d->ld_out_y % 4 == 0 && d->ld_out_y >= d->n_valid, "out_y unaligned");
   if (d->residual) GCB_CHECK_ARG(aligned16(d->residual) && d->ld_res % 4 == 0, "residual unaligned");
   GCB_CHECK_ARG(d->act == GCB_ACT_NONE || d->act == GCB_ACT_SWISH, "unknown activation");
+  GCB_CHECK_ARG(!(d->act == GCB_ACT_SWISH && d->ln_scale != nullptr),
+                "a layer is swish OR LayerNorm, not both");
   GCB_CHECK_ARG(d->n_pre_add >= 0 && d->n_pre_add <= 2, "n_pre_add must be 0..2");
   if (d->n_pre_add > 0) {
     GCB_CHECK_ARG(d->ln_scale == nullptr, "pre_add cannot be combined with LayerNorm");
@@ -191,9 +193,9 @@ int launch_tc_variant(const gcb_layer_desc& d, cudaStream_t stream) {
     max_clusters[dev][csize] = nc;
   }
   const int tiles = (d.rows + gcb::kTileM - 1) / gcb::kTileM;
-  // N-split schedule (n = 512, cluster of 2): one tile per cluster at a time; otherwise
-  // every CTA of the cluster has its own tile.
-  const bool nsplit = (csize == 2 && d.n == 512);
+  // N-split schedule (n = n_valid = 512, cluster of 2): one tile per cluster at a time;
+  // otherwise every CTA of the cluster has its own tile.  Same rule as in the kernel.
+  const bool nsplit = (csize == 2 && d.n == 512 && d.n_valid == 512);
   int clusters = nsplit ? tiles : (tiles + csize - 1) / csize;
   if (clusters > max_clusters[dev][csize]) clusters = max_clusters[dev][csize];
   cfg.gridDim = dim3(clusters * csize);
@@ -204,7 +206,6 @@ int launch_tc_variant(const gcb_layer_desc& d, cudaStream_t stream) {
 template <bool kSplit>
 int launch_tc(const gcb_layer_desc& d, cudaStream_t stream) {
   const bool swish = d.act == GCB_ACT_SWISH, ln = d.ln_scale != nullptr;
-  if (swish && ln) return launch_tc_variant<kSplit, true, true>(d, stream);
   if (swish) return launch_tc_variant<kSplit, true, false>(d, stream);
   if (ln) return launch_tc_variant<kSplit, false, true>(d, stream);
   return launch_tc_variant<kSplit, false, false>(d, stream);

@@ -715,27 +715,20 @@ mlp_chain_tc_kernel(const __grid_constant__ gcb_chain_desc d, const int nq, cons
       return g_count;
     };
 
-    auto unit_shifted_sums = [&](const float* s_bias, uint32_t taddr, float& shift, float& s1, float& s2) {
-      float p1 = 0.f, p2 = 0.f, q1 = 0.f, q2 = 0.f;
+    auto unit_stats = [&](const float* s_bias, uint32_t taddr, LnStats& st) {
       for (int c0 = 0; c0 < kUnitN; c0 += 32) {
         float v[32];
         ptx::tmem_ld32(taddr + c0, v);
-        float b[32];
+        if (s_bias != nullptr) {
+          float b[32];
 #pragma unroll
-        for (int q = 0; q < 8; ++q)
-          *reinterpret_cast<float4*>(&b[4 * q]) =
-              s_bias != nullptr ? *reinterpret_cast<const float4*>(s_bias + col_base + c0 + 4 * q)
-                                : make_float4(0.f, 0.f, 0.f, 0.f);
-        if (c0 == 0) shift = v[0] + b[0];
+          for (int q = 0; q < 8; ++q)
+            *reinterpret_cast<float4*>(&b[4 * q]) = *reinterpret_cast<const float4*>(s_bias + col_base + c0 + 4 * q);
 #pragma unroll
-        for (int j = 0; j < 32; j += 2) {
-          const float x0 = v[j] + b[j] - shift, x1 = v[j + 1] + b[j + 1] - shift;
-          p1 += x0; p2 = fmaf(x0, x0, p2);
-          q1 += x1; q2 = fmaf(x1, x1, q2);
+          for (int j = 0; j < 32; ++j) v[j] += b[j];
         }
+        st.add_block(v, 32);
       }
-      s1 = p1 + q1;
-      s2 = p2 + q2;
     };
 
     for (int st = 0; st < nsteps; ++st) {
@@ -794,10 +787,10 @@ mlp_chain_tc_kernel(const __grid_constant__ gcb_chain_desc d, const int nq, cons
         const uint32_t taddr = tmem_base + lane_base + buf * kUnitN;
         if (kind >= kKindLN) {
           const uint32_t lb = ln_count & 1, par = (ln_count >> 1) & 1;
-          float shift, s1, s2;
-          unit_shifted_sums(cx.s_bias, taddr, shift, s1, s2);
-          const float mean_h = shift + s1 * (1.0f / kUnitN);
-          const float m2_h = fmaxf(s2 - s1 * s1 * (1.0f / kUnitN), 0.f);
+          LnStats st;
+          unit_stats(cx.s_bias, taddr, st);
+          const float mean_h = st.shift + st.mean;
+          const float m2_h = st.m2;
           const int myrow = ew * 32 + lane;
           // (with two epilogue groups both compute the statistics of all 256 columns and run
           // their own exchange with the same group of the partner CTA: no coupling between groups)

@@ -5,13 +5,13 @@
 // One persistent 512-thread CTA per SM.  Work is cut into UNITS of 128 rows x 256 output
 // columns; TMEM holds TWO 128x256 fp32 accumulators, so the epilogue of unit u overlaps
 // the MMAs of unit u+1.  Two schedules:
-//   N-split (n = 512, cluster of 2): both CTAs of the cluster work on the SAME 128-row
+//   N-split (n = n_valid = 512, cluster of 2): both CTAs of the cluster work on the SAME 128-row
 //     tile, CTA r owning output columns [256r, 256r+256).  The A block of every K-step is
 //     fetched once and multicast to both CTAs, each CTA streams only its half of the
 //     weights, and LayerNorm row statistics are combined across the pair through
 //     distributed shared memory.  Consecutive units of a CTA are consecutive tiles.
-//   unsplit (n = 256, or cluster of 1): every CTA walks its own tiles (n/256 units per
-//     tile); the CTAs of a cluster share the weight stream by multicast.
+//   unsplit (n = 256, n_valid < 512, or a cluster of 1 or 4): every CTA walks its own tiles
+//     (n/256 units per tile); the CTAs of a cluster share the weight stream by multicast.
 // Warp roles:
 //   warp 0        TMA lane: per K-step streams (a) 1/cluster of the pre-packed bf16 weight
 //                 tile with cp.async.bulk, multicast to every CTA of the cluster, and (b)
@@ -93,6 +93,58 @@ __device__ __forceinline__ float swish_f(float x) {
   // branch-free (~2 ulp), so 32 independent elements pipeline through the SFU.
   return __fdividef(x, 1.0f + __expf(-x));
 }
+
+// LayerNorm statistics of one row, fed one 32-column block (one tcgen05.ld) at a time in
+// column order.  Each block's mean and M2 are taken in two passes over its registers, around
+// `shift` = the mean of the row's first block, and the blocks are merged with Chan's update.
+// A one-pass s2 - s1^2 / n around a single column cancels when that column lies far from
+// the row mean; this stays accurate wherever an outlier sits.  The layer and the chain
+// kernel both use it, so their results stay bit-identical.  The divisions are approximate
+// (exact for the power-of-two counts of full blocks): an IEEE division's slow-path call
+// costs the epilogue registers it does not have.
+struct LnStats {
+  float shift = 0.f;   // the row's values are x - shift below
+  float mean = 0.f;    // mean of (x - shift) over the columns added so far
+  float m2 = 0.f;      // sum of squared deviations from the mean
+  float cnt = 0.f;     // columns added so far
+
+  // x: the block's pre-LayerNorm values (overwritten); its first nv (1..32) are valid.
+  __device__ __forceinline__ void add_block(float (&x)[32], int nv) {
+    const float nb = static_cast<float>(nv);
+    if (cnt == 0.f) {
+      float p = 0.f, q = 0.f;                      // two chains for ILP
+#pragma unroll
+      for (int j = 0; j < 32; j += 2) {
+        if (j < nv) p += x[j];
+        if (j + 1 < nv) q += x[j + 1];
+      }
+      shift = __fdividef(p + q, nb);
+    }
+    float p = 0.f, q = 0.f;
+#pragma unroll
+    for (int j = 0; j < 32; j += 2) {
+      x[j] -= shift;
+      x[j + 1] -= shift;
+      if (j < nv) p += x[j];
+      if (j + 1 < nv) q += x[j + 1];
+    }
+    const float mb = __fdividef(p + q, nb);
+    p = 0.f;
+    q = 0.f;
+#pragma unroll
+    for (int j = 0; j < 32; j += 2) {
+      const float d0 = x[j] - mb, d1 = x[j + 1] - mb;
+      if (j < nv) p = fmaf(d0, d0, p);
+      if (j + 1 < nv) q = fmaf(d1, d1, q);
+    }
+    const float n = cnt + nb;
+    const float f = __fdividef(nb, n);
+    const float d = mb - mean;
+    mean = fmaf(d, f, mean);
+    m2 += fmaf(d * d, cnt * f, p + q);
+    cnt = n;
+  }
+};
 
 // Optional timeline trace (debug): when non-null, CTA 0 records clock64() at a few
 // points of each of its first kTraceTiles units; see gcb_debug_trace in api.cu.
@@ -189,7 +241,9 @@ mlp_layer_tc_kernel(const __grid_constant__ gcb_layer_desc d) {
   // tiles in lockstep and share every weight tile through TMA multicast.
   const uint32_t crank = ptx::cluster_ctarank();
   const uint32_t csize = ptx::cluster_nctarank();
-  const bool nsplit = (csize == 2) && (n_halves == 2);
+  // N-split only for full 512-wide rows: its LayerNorm statistics are over all 256 columns
+  // of each half, and it stores whole halves.  Any other n = 512 layer runs unsplit.
+  const bool nsplit = (csize == 2) && (n_halves == 2) && (d.n_valid == n);
   const uint32_t tiles_per_iter = nsplit ? 1u : csize;       // tiles a cluster covers per iteration
   const uint32_t tile_first = ptx::cluster_id_x() * tiles_per_iter;
   const uint32_t tile_stride = ptx::num_clusters_x() * tiles_per_iter;
@@ -386,9 +440,8 @@ mlp_layer_tc_kernel(const __grid_constant__ gcb_layer_desc d) {
     const int rsub = lane >> 3;                  // row within a group of 4
     uint32_t g_count = 0;
 
-    // LayerNorm statistics of one unit: shifted sums over its valid columns.
-    auto stats_unit = [&](uint32_t taddr, int col_base, int ncols, float& shift, float& s1,
-                          float& s2, bool first) {
+    // LayerNorm statistics of one unit's valid columns, added to those of the earlier units.
+    auto stats_unit = [&](uint32_t taddr, int col_base, int ncols, LnStats& st) {
       for (int c0 = 0; c0 < ncols; c0 += 32) {
         float v[32];
         ptx::tmem_ld32(taddr + c0, v);
@@ -397,26 +450,10 @@ mlp_layer_tc_kernel(const __grid_constant__ gcb_layer_desc d) {
         for (int q = 0; q < 8; ++q)
           *reinterpret_cast<float4*>(&b[4 * q]) =
               *reinterpret_cast<const float4*>(s_bias + col_base + c0 + 4 * q);
-        if (first && c0 == 0) shift = v[0] + b[0];
-        if (c0 + 32 <= ncols) {
-          float p1 = 0.f, p2 = 0.f, q1 = 0.f, q2 = 0.f;   // two chains for ILP
 #pragma unroll
-          for (int j = 0; j < 32; j += 2) {
-            const float x0 = v[j] + b[j] - shift, x1 = v[j + 1] + b[j + 1] - shift;
-            p1 += x0; p2 = fmaf(x0, x0, p2);
-            q1 += x1; q2 = fmaf(x1, x1, q2);
-          }
-          s1 += p1 + q1; s2 += p2 + q2;
-        } else {
-#pragma unroll
-          for (int j = 0; j < 32; ++j) {
-            if (c0 + j < ncols) {
-              const float x = v[j] + b[j] - shift;
-              s1 += x;
-              s2 = fmaf(x, x, s2);
-            }
-          }
-        }
+        for (int j = 0; j < 32; ++j) v[j] += b[j];
+        if (c0 + 32 <= ncols) st.add_block(v, 32);
+        else st.add_block(v, ncols - c0);
       }
     };
 
@@ -568,30 +605,6 @@ mlp_layer_tc_kernel(const __grid_constant__ gcb_layer_desc d) {
       if (lane == 0) ptx::mbar_arrive(&tmem_empty_bar[buf]);
     };
 
-    // One pass over a full 256-column unit: shifted sums  s1 = sum(x - shift),
-    // s2 = sum((x - shift)^2)  with shift = the row's first value of this unit.
-    auto unit_shifted_sums = [&](uint32_t taddr, int col_base, float& shift, float& s1, float& s2) {
-      float p1 = 0.f, p2 = 0.f, q1 = 0.f, q2 = 0.f;     // two chains for ILP
-      for (int c0 = 0; c0 < kUnitN; c0 += 32) {
-        float v[32];
-        ptx::tmem_ld32(taddr + c0, v);
-        float b[32];
-#pragma unroll
-        for (int q = 0; q < 8; ++q)
-          *reinterpret_cast<float4*>(&b[4 * q]) =
-              *reinterpret_cast<const float4*>(s_bias + col_base + c0 + 4 * q);
-        if (c0 == 0) shift = v[0] + b[0];
-#pragma unroll
-        for (int j = 0; j < 32; j += 2) {
-          const float x0 = v[j] + b[j] - shift, x1 = v[j + 1] + b[j + 1] - shift;
-          p1 += x0; p2 = fmaf(x0, x0, p2);
-          q1 += x1; q2 = fmaf(x1, x1, q2);
-        }
-      }
-      s1 = p1 + q1;
-      s2 = p2 + q2;
-    };
-
     uint32_t u = 0;
     for (uint32_t base = tile_first; base < static_cast<uint32_t>(num_tiles); base += tile_stride) {
       const uint32_t tile = base + tile_off;
@@ -619,10 +632,10 @@ mlp_layer_tc_kernel(const __grid_constant__ gcb_layer_desc d) {
         if (ew == 0 && lane == 0) trace(u, 3);
         const int col_base = static_cast<int>(crank) * kUnitN;
         const uint32_t taddr = tmem_base + lane_base + buf * kUnitN;
-        float shift, s1, s2;
-        unit_shifted_sums(taddr, col_base, shift, s1, s2);
-        const float mean_h = shift + s1 * (1.0f / kUnitN);              // mean of my 256 columns
-        const float m2_h = fmaxf(s2 - s1 * s1 * (1.0f / kUnitN), 0.f);  // sum of squared deviations
+        LnStats st;
+        stats_unit(taddr, col_base, kUnitN, st);
+        const float mean_h = st.shift + st.mean;                        // mean of my 256 columns
+        const float m2_h = st.m2;                                       // sum of squared deviations
         const int myrow = ew * 32 + lane;
         const uint32_t peer = crank ^ 1u;
         ptx::st_async_f32x2(ptx::mapa(ptx::smem_addr(&s_lnx[buf * kTileM + myrow]), peer), mean_h, m2_h,
@@ -642,7 +655,7 @@ mlp_layer_tc_kernel(const __grid_constant__ gcb_layer_desc d) {
       } else {
         // Statistics over all units of the row (overlapping the MMAs of the later ones),
         // then normalise / store unit by unit, releasing each accumulator as soon as done.
-        float shift = 0.f, s1 = 0.f, s2 = 0.f;
+        LnStats st;
         const uint32_t u0 = u;
         for (int h = 0; h < n_halves; ++h, ++u) {
           const uint32_t buf = u & 1;
@@ -650,14 +663,11 @@ mlp_layer_tc_kernel(const __grid_constant__ gcb_layer_desc d) {
           ptx::tc_fence_after_sync();
           if (ew == 0 && lane == 0) trace(u, 3);
           const int col_base = h * kUnitN;
-          stats_unit(tmem_base + lane_base + buf * kUnitN, col_base, min(kUnitN, n_valid - col_base),
-                     shift, s1, s2, h == 0);
+          stats_unit(tmem_base + lane_base + buf * kUnitN, col_base, min(kUnitN, n_valid - col_base), st);
           if (ew == 0 && lane == 0) trace(u, 4);
         }
-        const float inv_n = 1.0f / static_cast<float>(n_valid);
-        const float m1 = s1 * inv_n;
-        const float mean = shift + m1;
-        const float rstd = rsqrtf(fmaxf(s2 * inv_n - m1 * m1, 0.f) + 1e-5f);
+        const float mean = st.shift + st.mean;
+        const float rstd = rsqrtf(st.m2 * (1.0f / static_cast<float>(n_valid)) + 1e-5f);
         for (int h = 0; h < n_halves; ++h) {
           const uint32_t uu = u0 + h, buf = uu & 1;
           const int col_base = h * kUnitN;

@@ -83,6 +83,8 @@ typedef struct {
  *     z   = concat(segments)                         [rows, K],  K = sum k
  *     y   = act(z @ W + bias + sum_p pre_add_p)      [rows, n]
  *     y   = LayerNorm(y) * ln_scale + ln_offset      (if ln_scale != NULL; eps 1e-5)
+ * A layer has either the swish activation or LayerNorm, not both (GCB_ERR_INVALID);
+ * LayerNorm statistics are over the n_valid columns.
  *     out_y[r] = y[r]                                (if out_y  != NULL)
  *     out[r]   = (residual ? residual[r] : 0) + y[r] (if out    != NULL)
  * Replaces one hk.Linear (+ jax.nn.swish | + hk.LayerNorm + residual add) of

@@ -2,9 +2,24 @@
 import functools
 
 import numpy as np
+import pytest
 
 from graphcast_b200 import graph as graph_lib
 from oracle import gnn as oracle_gnn
+
+
+@pytest.fixture
+def cluster(request):
+  """CTAs per cluster of the tensor-core layer kernel for one test (parametrize it with
+  indirect=True).  The setting is process-global, so the library default of 2 is restored
+  however the test ends: a leaked value would move every later test onto another schedule."""
+  from graphcast_b200 import _native
+  lib = _native.lib()
+  _native.check(lib.gcb_set_cluster_size(request.param), "gcb_set_cluster_size")
+  try:
+    yield request.param
+  finally:
+    _native.check(lib.gcb_set_cluster_size(2), "gcb_set_cluster_size")
 
 
 @functools.lru_cache(maxsize=None)

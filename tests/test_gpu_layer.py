@@ -7,6 +7,7 @@ import numpy as np
 import pytest
 import torch
 
+from _cases import cluster  # noqa: F401  (fixture)
 from graphcast_b200 import _native
 
 pytestmark = pytest.mark.gpu
@@ -128,7 +129,11 @@ def test_fan_in_three_segment(prec):
   assert err < TOL[prec], err
 
 
-@pytest.mark.parametrize("rows", [1, 127, 128, 129, 148 * 128 + 5])
+# 5 * 128 + 1 rows at a cluster of 4: one full cluster, then one with two idle CTAs
+RAGGED_ROWS = [1, 127, 128, 129, 5 * 128 + 1, 148 * 128 + 5]
+
+
+@pytest.mark.parametrize("rows", RAGGED_ROWS)
 def test_ragged_row_counts(rows):
   err = _run_case("bf16x3", rows=rows, segs=[(max(rows, 1), 512, 512, False, 1)], n=512,
                   n_valid=512, act=False, ln=True, residual=True, out_y=False)
@@ -297,3 +302,32 @@ def test_tensor_path_matches_simt_arm_selftest():
     err = C.c_float(-1)
     assert lib.gcb_selftest_layer(3000, 1024, 512, _native.PRECISIONS[prec], C.byref(err)) == 0
     assert 0 <= err.value < tol
+
+
+# The tests above run at the library's default cluster size of 2 (the N-split schedule for
+# n = 512).  Clusters of 1 and 4 take the unsplit schedule: each CTA owns its tiles and runs
+# both 256-column units, the weight stream is multicast to 4 CTAs, and some clusters have
+# idle CTAs.  The fp32 CUDA-core arm has no clusters, so only the tensor-core precisions repeat.
+@pytest.mark.parametrize("cluster", [1, 4], indirect=True)
+@pytest.mark.parametrize("rows", RAGGED_ROWS)
+def test_ragged_row_counts_at_cluster_size(rows, cluster):
+  test_ragged_row_counts(rows)
+
+
+@pytest.mark.parametrize("cluster", [1, 4], indirect=True)
+def test_padded_inputs_and_narrow_output_at_cluster_size(cluster):
+  test_padded_inputs_and_narrow_output("bf16x3")
+
+
+@pytest.mark.parametrize("cluster", [1, 4], indirect=True)
+@pytest.mark.parametrize("prec", ["bf16x3", "bf16"])
+@pytest.mark.parametrize("rows", [700, 128 * 148 + 77])
+def test_gathered_pre_activation_addends_at_cluster_size(prec, rows, cluster):
+  test_gathered_pre_activation_addends(prec, rows)
+
+
+@pytest.mark.parametrize("cluster", [1, 4], indirect=True)
+@pytest.mark.parametrize("prec", ["bf16x3", "bf16"])
+@pytest.mark.parametrize("rows", [1, 333, 128 * 148 * 2 + 5])
+def test_operand_image_chain_at_cluster_size(prec, rows, cluster):
+  test_operand_image_chain(prec, rows)
